@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W  # N-axis sharded over N GPUs
     python bench.py --impl reference --steps 2 --warmup 1          # reference algorithm on the host cores
+    python bench.py --steps 50 --warmup 5 --dump-outputs DIR       # + what the timed loop computed, as DIR/*.npy
 
 One step = get_next_item_to_label() -> oracle(idx) -> add_label() -> get_best_model_prediction()
 (reference main.py:91-94).  Workload: synthetic M=256, N=1e6, C=100 (BASELINE.json configs[2]),
@@ -62,7 +63,32 @@ def parse():
     ap.add_argument("--dense", action="store_true", help="worst-case synthetic slab (wrong class uniform)")
     ap.add_argument("--no-dense-extra", dest="dense_extra", action="store_false",
                     help="skip the dense worst-case slab that the N=1 run reports under modes.dense_slab")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the device loop computed as DIR/<name>.npy (rank 0)")
     return ap.parse_args()
+
+
+DUMP_ARRAY_BYTES = 16 << 20     # per array: with three item- or class-sized arrays a dump stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every tensor as ``out_dir/<name>.npy``: floating point as float32 (float64 stays), integers as float64.
+    Larger than DUMP_ARRAY_BYTES, an array is replaced by a fixed, seeded sample of its rows (all axes but the last
+    flattened), and the row numbers go to ``<name>_rows.npy``: two builds given the same arguments sample the same
+    rows, so their dumps compare element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = torch.as_tensor(t)
+        t = t.float() if t.is_floating_point() and t.dtype != torch.float64 else t.double()
+        rows = t.reshape(-1, t.shape[-1]) if t.dim() > 1 else t.reshape(-1, 1)
+        if rows.numel() * rows.element_size() > DUMP_ARRAY_BYTES:
+            k = max(1, DUMP_ARRAY_BYTES // (rows.shape[1] * rows.element_size()))
+            pick = np.sort(np.random.default_rng(0).choice(rows.shape[0], size=k, replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), pick.astype(np.float64))
+            t = rows[torch.from_numpy(pick).to(rows.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -495,6 +521,14 @@ def main():
     value = args.steps / (ms / 1e3)
     picks_dev = sel.history()[0][-(args.steps):].tolist()
     ties_dev = int(sel.history()[2].sum())
+    if args.dump_outputs:
+        if rank == 0:   # with several ranks, eig and pi_hat_xi are rank 0's shard of the item axis
+            h_idx, h_q, h_tie = sel.history()
+            dump_outputs(args.dump_outputs, {
+                "history_idx": h_idx[-args.steps:], "history_q": h_q[-args.steps:], "history_tie": h_tie[-args.steps:],
+                "best_model": eng.best_model[:1], "pbest": sel.get_pbest(),
+                "pi_hat": sel.pi_hat, "dirichlets": sel.dirichlets, "eig": sel.eig, "pi_hat_xi": sel.pi_hat_xi})
+        barrier()
 
     prof_steps = min(10, args.steps)
     prof = eager_profile(sel, labels_dev, prof_steps)

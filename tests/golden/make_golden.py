@@ -23,6 +23,8 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))
+from helpers import final_dirichlets  # noqa: E402
 
 REF = os.environ.get("CODA_REFERENCE_PATH", "/root/reference")
 
@@ -53,7 +55,7 @@ def seed_all(seed):
     torch.manual_seed(seed)
 
 
-def run_case(ref_coda, name, H, N, C, data_seed, steps, dense=False, ctor=None, save_eig=True, slim=False):
+def run_case(ref_coda, name, H, N, C, data_seed, steps, dense=False, ctor=None, save_eig=True, slim=False, drop=()):
     from coda_b200.synth import synth
     ctor = ctor or {}
     preds, labels = synth(H, N, C, data_seed, dense=dense)
@@ -114,6 +116,10 @@ def run_case(ref_coda, name, H, N, C, data_seed, steps, dense=False, ctor=None, 
         for k in ("init_dirichlets", "final_dirichlets", "init_pi_hat_xi"):
             out.pop(k)
         out["xi_head"] = out["xi_head"][:, :8]
+    elif np.array_equal(final_dirichlets(out), out["final_dirichlets"]):
+        out.pop("final_dirichlets")          # tests/helpers.py rebuilds it from init_dirichlets and dir_row
+    for k in drop:
+        out.pop(k)
     path = os.path.join(HERE, name + ".npz")
     np.savez_compressed(path, **out)
     print(name, "idx", idxs, "ties", ntie, "->", path, os.path.getsize(path) // 1024, "KiB")
@@ -132,10 +138,45 @@ def unit_vectors(ref_coda):
     print("quadrature_kat", out[0])
 
 
+def _rng_state():
+    version, words, gauss = random.getstate()
+    assert version == 3 and gauss is None
+    return np.array(words, dtype=np.uint32)
+
+
+def acquisitions(ref_coda):
+    """The ablation acquisitions q='iid' / 'uncertainty' (coda.py:287-295) and the --prefilter-n subsample
+    (coda.py:221-223): per step the pick, its score, the Python RNG state right after the pick (what random.choice /
+    random.sample consumed) and the best model after the label."""
+    from coda_b200.synth import synth
+    out = {}
+    preds, labels = synth(12, 500, 6, seed=17)
+    for q in ("iid", "uncertainty"):
+        random.seed(4)
+        sel = ref_coda.CODA(_DS(preds, labels), q=q)
+        idx, qs, states, bests = [], [], [], []
+        for _ in range(4):
+            i, v = sel.get_next_item_to_label()
+            states.append(_rng_state())
+            sel.add_label(i, int(labels[i]), v)
+            idx.append(i); qs.append(v); bests.append(int(sel.get_best_model_prediction()))
+        out.update({f"{q}_idx": np.array(idx), f"{q}_q": np.array(qs, dtype=np.float64),
+                    f"{q}_rng": np.stack(states), f"{q}_best_model": np.array(bests)})
+    preds, labels = synth(10, 600, 6, seed=8)
+    random.seed(5)
+    sel = ref_coda.CODA(_DS(preds, labels), prefilter_n=50)
+    i, v = sel.get_next_item_to_label()
+    out.update(prefilter_idx=np.array(i), prefilter_q=np.array(v, dtype=np.float64), prefilter_rng=_rng_state(),
+               prefilter_stochastic=np.array(int(sel.stochastic)))
+    path = os.path.join(HERE, "acquisitions.npz")
+    np.savez_compressed(path, **out)
+    print("acquisitions", {k: v.tolist() for k, v in out.items() if not k.endswith("_rng")}, "->", path)
+
+
 if __name__ == "__main__":
     ref = import_reference()
     unit_vectors(ref)
-    which = sys.argv[1:] or ["tiny", "small", "c100", "dense", "nodiag"]
+    which = sys.argv[1:] or ["tiny", "small", "c100", "dense", "nodiag", "acq"]
     if "tiny" in which:
         run_case(ref, "traj_tiny_h8_n300_c5", 8, 300, 5, 1, steps=6)
     if "small" in which:
@@ -149,5 +190,7 @@ if __name__ == "__main__":
                  ctor=dict(disable_diag_prior=1, alpha=0.8, learning_rate=0.05, multiplier=1.5))
     if "h256" in which:   # full-width tensor-core tile (Hp = 256, C = 100): ~6 min per step on 8 cores
         run_case(ref, "traj_h256_h256_n1500_c100", 256, 1500, 100, 5, steps=2, slim=True)
-    if "cfg2" in which:   # ~270 s/step on 8 cores: a few steps only
-        run_case(ref, "traj_cfg2_h64_n50000_c10", 64, 50000, 10, 0, steps=3)
+    if "cfg2" in which:   # ~270 s/step on 8 cores: a few steps only; no test reads the 2 MB initial pi_hat_xi
+        run_case(ref, "traj_cfg2_h64_n50000_c10", 64, 50000, 10, 0, steps=3, drop=("init_pi_hat_xi",))
+    if "acq" in which:
+        acquisitions(ref)

@@ -25,7 +25,18 @@ def load_golden(name):
     g["ctor"] = {}
     for k, v in zip(g["ctor_keys"].tolist(), g["ctor_vals"].tolist()):
         g["ctor"][k] = bool(v) if k == "disable_diag_prior" else (int(v) if k == "prefilter_n" else float(v))
+    if "final_dirichlets" not in g and "init_dirichlets" in g:
+        g["final_dirichlets"] = final_dirichlets(g)
     return g
+
+
+def final_dirichlets(g):
+    """The posterior after the trajectory: a label of class t rewrites only dirichlets[:, t] (coda.py:316-317), and
+    dir_row holds that column after every step, so a fixture need not store the whole H x C x C array twice."""
+    d = g["init_dirichlets"].copy()
+    for k, i in enumerate(g["idx"]):
+        d[:, g["labels"][i]] = g["dir_row"][k]
+    return d
 
 
 def golden_slab(g):
