@@ -91,6 +91,14 @@ SIGNATURES = {
     "coda_b200_pi_reduce": (i32, [p, i64, i32, i32, p, p, p, p]),
     "coda_b200_shadow_build": (i32, [p, i64, i32, i64, i32, p, i32, i64, p, p]),
     "coda_b200_pi_rank1": (i32, [p, p, i32, i64, i32, p, f64, i32, p, p, p, p, i32, i32, p]),
+    "coda_b200_scan_slab_f16": (i32, [p, i64, i32, i64, i32, p, p, p, p, p, p]),
+    "coda_b200_confusion_accum_f16": (i32, [p, i64, p, i32, i64, i32, i32, p, p]),
+    "coda_b200_confusion_sorted_f16": (i32, [p, i64, p, p, i32, i64, i32, i32, p, p]),
+    "coda_b200_pi_full_f16": (i32, [p, i64, p, i32, i64, i32, p, p]),
+    "coda_b200_pi_full_tc_ok_f16": (i32, [i32, i64, i32, i64]),
+    "coda_b200_pi_full_tc_f16": (i32, [p, i64, p, i32, i64, i32, p, p, p, p]),
+    "coda_b200_shadow_build_f16": (i32, [p, i64, i32, i64, i32, p, i32, i64, p, p]),
+    "coda_b200_pi_rank1_f16": (i32, [p, p, i32, i64, i32, p, f64, i32, p, p, p, p, i32, i32, p]),
     "coda_b200_tables_scratch_bytes": (sz, [i32, i32]),
     "coda_b200_beta_tables": (i32, [p, p, i32, i32, i32, f64, i32, i32, p, p, p, p, p, p, p, p, p, p]),
     "coda_b200_pair_count": (i32, [p, i32, i64, i32, p, p, p, p]),

@@ -1,5 +1,6 @@
 // Shared device/host helpers for the coda_b200 kernels (sm_100a only).
 #pragma once
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -133,6 +134,34 @@ __device__ __forceinline__ void tma_load_1d(void* smem_dst, const void* gmem_src
           smem_u32(smem_dst)),
       "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar))
       : "memory");
+}
+
+// ---- slab element type: fp32, or IEEE binary16 (`__half`) converted on load -------------------------------------
+// Every kernel that reads the prediction slab computes in fp32.  The fp16 -> fp32 conversion is exact, so a kernel
+// instantiated for a 16-bit slab does the same arithmetic, with the same bits, as its fp32 twin on the upcast slab.
+__device__ __forceinline__ float slab_ld(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float slab_ld(const __half* p) { return __half2float(__ldg(p)); }
+__device__ __forceinline__ float slab_f(float v) { return v; }
+__device__ __forceinline__ float slab_f(__half v) { return __half2float(v); }
+
+// Bulk copies of 16-bit slab ranges: the range's start and length need not be 16-byte aligned, so the 16-byte aligned
+// window around it is copied and the range starts `slab_head` bytes into the window.  The window stays inside the
+// 16-byte granules of the allocation (device allocations are at least 256-byte aligned and sized).  Shared-memory
+// buffers that receive such a window carry SLAB_PAD bytes of slack.  An fp32 range is copied as is (callers guarantee
+// its alignment), so the fp32 instantiations issue exactly the copies they always did.
+template <typename T>
+__host__ __device__ constexpr uint32_t slab_pad() { return sizeof(T) == 4 ? 0u : 16u; }
+template <typename T>
+__device__ __forceinline__ uint32_t slab_head(const T* p) {
+  return sizeof(T) == 4 ? 0u : (uint32_t)(reinterpret_cast<uintptr_t>(p) & 15);
+}
+template <typename T>
+__device__ __forceinline__ uint32_t tma_load_slab(void* smem_dst, const T* src, uint32_t bytes, uint64_t* bar) {
+  const uint32_t head = slab_head(src);
+  const uint32_t win = sizeof(T) == 4 ? bytes : ((head + bytes + 15u) & ~15u);
+  mbar_expect_tx(bar, win);
+  tma_load_1d(smem_dst, reinterpret_cast<const unsigned char*>(src) - head, win, bar);
+  return head;
 }
 
 // ---- arg-max records ---------------------------------------------------------------------------

@@ -23,6 +23,12 @@
 //                                       one tcgen05.commit per chunk frees its A and D slots
 //   warps 4..19       drain             tcgen05.ld of both accumulators every G models, final store of U
 //   warps 20..31      converters        fp32 staging -> fp16 hi / lo limbs in the UMMA K-major core-matrix order
+//
+// An fp16 slab (k_pi_full_tc<__half>) is staged as fp16, half the bytes per unit.  Its values ARE their own hi limb and
+// their lo limb is exactly 0 (the split of the fp32 upcast gives the same two limbs), so the converters only repack the
+// fp16 items into the core-matrix order; the lo limbs of the A ring are zeroed once and every MMA is issued as for fp32:
+// the result has the bits of the fp32 pass on the upcast slab.  Its units are copied as 16-byte aligned windows
+// (common.cuh: tma_load_slab), so an item-range view or an odd N needs no alignment beyond 8 bytes.
 // The kernel lives on bytes in flight: every (tile, model) pulls 51 KB of slab from HBM and 50 KB of D limbs from L2, so
 // shared memory is split between the fp32 staging ring and a deep D ring; the converted A chunks only need a short ring.
 // Every wait is bounded: a pipeline that stops sets CODA_B200_FLAG_PIPELINE_TIMEOUT and the kernel drains out.
@@ -49,8 +55,8 @@ constexpr float PT_LO_SCALE = 4096.f;     // lo limbs are stored times 2^12
 constexpr long long PT_TIMEOUT_CYCLES = 4000000000LL;   // ~2 s
 
 struct PiTcArgs {
-  const float* preds;
-  long long ldh;              // floats between models
+  const void* preds;          // float or __half [H][N][C]
+  long long ldh;              // elements between models
   const unsigned char* wb;    // [H][KC][2 k_cores][2 Np/8 (hi | lo)][8][8] fp16, then the 16-byte header (max |D| bits)
   const uint32_t* dmax;       // header: bits of max |D|
   float* U;
@@ -211,6 +217,7 @@ __global__ void __launch_bounds__(256) k_pi_w_limbs(const float* __restrict__ D,
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(PT_THREADS, 1) k_pi_full_tc(PiTcArgs a) {
   extern __shared__ __align__(1024) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -219,7 +226,8 @@ __global__ void __launch_bounds__(PT_THREADS, 1) k_pi_full_tc(PiTcArgs a) {
   const int cnt = (int)min((long long)PT_M, a.N - n0);
 
   // ---- shared memory carve-up ----------------------------------------------------------------------
-  const uint32_t stage_bytes = (uint32_t)PT_HALF * C * 4u;                    // fp32 block of one (model, 32-item quarter)
+  const T* preds = reinterpret_cast<const T*>(a.preds);
+  const uint32_t stage_bytes = (uint32_t)PT_HALF * C * sizeof(T) + slab_pad<T>();   // block of one (model, 32-item quarter)
   const uint32_t stage_stride = (stage_bytes + 127u) & ~127u;
   const uint32_t a_limb = (uint32_t)PT_M * 16u * 2u;                          // 4 KB: one limb of one A chunk
   const uint32_t b_limb = (uint32_t)Np * 16u * 2u;                            // one limb of one D chunk
@@ -252,6 +260,13 @@ __global__ void __launch_bounds__(PT_THREADS, 1) k_pi_full_tc(PiTcArgs a) {
     *abort_s = (*a.flags & CODA_B200_FLAG_PIPELINE_TIMEOUT) ? 1 : 0;          // an earlier CTA already gave up
     mbar_fence_init();
   }
+  if constexpr (sizeof(T) == 2) {                                              // fp16 slab: the lo limbs of A are 0
+    for (uint32_t i = tid; i < (uint32_t)SA * (a_limb / 16u); i += PT_THREADS) {
+      const uint32_t s = i / (a_limb / 16u), e = i % (a_limb / 16u);
+      *reinterpret_cast<uint4*>(aslots + (size_t)s * 2u * a_limb + a_limb + e * 16u) = make_uint4(0u, 0u, 0u, 0u);
+    }
+    pt_fence_proxy_async();                                                    // visible to the tensor core
+  }
   if (warp == 3) {
     __syncwarp();
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u)
@@ -277,10 +292,9 @@ __global__ void __launch_bounds__(PT_THREADS, 1) k_pi_full_tc(PiTcArgs a) {
           pt_arrive(&fullS[r.slot]);
           continue;
         }
-        const uint32_t bytes = (uint32_t)items * C * 4u;
-        mbar_expect_tx(&fullS[r.slot], bytes);
-        tma_load_1d(stage0 + (size_t)r.slot * stage_stride,
-                    a.preds + (size_t)(j / PT_WARPS_PER_CHUNK) * a.ldh + (size_t)(n0 + hf * PT_HALF) * C, bytes, &fullS[r.slot]);
+        const uint32_t bytes = (uint32_t)items * C * sizeof(T);
+        tma_load_slab(stage0 + (size_t)r.slot * stage_stride,
+                      preds + (size_t)(j / PT_WARPS_PER_CHUNK) * a.ldh + (size_t)(n0 + hf * PT_HALF) * C, bytes, &fullS[r.slot]);
       }
     }
   } else if (warp == 1) {
@@ -407,7 +421,10 @@ __global__ void __launch_bounds__(PT_THREADS, 1) k_pi_full_tc(PiTcArgs a) {
       ok = pt_wait(&fullS[rs.slot], rs.ph, abort_s);
       ok = __all_sync(CODA_FULL, ok);
       if (!ok) break;
-      const float* src = reinterpret_cast<const float*>(stage0 + (size_t)rs.slot * stage_stride);
+      const unsigned char* stage = stage0 + (size_t)rs.slot * stage_stride;
+      const float* src = reinterpret_cast<const float*>(stage);
+      // fp16: the unit starts `head` bytes into its window; every row of an eligible view is 8-byte aligned
+      const unsigned char* src16 = stage + slab_head(preds + (size_t)h * a.ldh + (size_t)(n0 + sub * PT_HALF) * C);
       for (; q < (h + 1) * KC; q += PT_CONV_GROUPS, ra.step(PT_CONV_GROUPS, SA)) {
         const int kc = q - h * KC;
         const int w = q - SA;                                 // the chunk that held this A slot
@@ -417,6 +434,26 @@ __global__ void __launch_bounds__(PT_THREADS, 1) k_pi_full_tc(PiTcArgs a) {
           if (!ok) break;
         }
         unsigned char* dst = aslots + (size_t)ra.slot * 2u * a_limb;
+        if constexpr (sizeof(T) == 2) {
+          uint2 v[PT_HALF / 32][4];                           // 4 x 4 halves = the 16 columns of this chunk
+#pragma unroll
+          for (int it = 0; it < PT_HALF / 32; ++it) {
+            const unsigned char* rowp = src16 + ((size_t)(it * 32 + lane) * C + kc * 16) * 2u;
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+              v[it][j] = (kc * 16 + j * 4 < C) ? *reinterpret_cast<const uint2*>(rowp + j * 8) : make_uint2(0u, 0u);
+          }
+#pragma unroll
+          for (int it = 0; it < PT_HALF / 32; ++it) {
+            const int item = sub * PT_HALF + it * 32 + lane;
+#pragma unroll
+            for (int kcore = 0; kcore < 2; ++kcore) {
+              const uint2 x = v[it][2 * kcore], y = v[it][2 * kcore + 1];
+              const uint32_t off = (uint32_t)((kcore * (PT_M / 8) + (item >> 3)) * 128 + (item & 7) * 16);
+              *reinterpret_cast<uint4*>(dst + off) = make_uint4(x.x, x.y, y.x, y.y);
+            }
+          }
+        } else {
         // all loads first: the limb stores below go to shared memory too, so the compiler would not hoist loads over them
         float4 v[PT_HALF / 32][2][2];
 #pragma unroll
@@ -443,6 +480,7 @@ __global__ void __launch_bounds__(PT_THREADS, 1) k_pi_full_tc(PiTcArgs a) {
             *reinterpret_cast<uint4*>(dst + a_limb + off) = lo;
           }
         }
+        }
         pt_fence_proxy_async();
         __syncwarp();
         if (lane == 0) pt_arrive(&fullK[q & (PT_CHUNK_BARS - 1)]);
@@ -466,9 +504,9 @@ struct PiTcPlan {
 };
 
 // shared-memory split: a short ring of converted A chunks, the rest shared between slab staging and D chunks in flight
-PiTcPlan pi_tc_plan(int C, int Np) {
+PiTcPlan pi_tc_plan(int C, int Np, size_t esize) {
   const size_t budget = 227 * 1024;
-  const size_t stage = ((size_t)PT_HALF * C * 4 + 127) & ~(size_t)127;
+  const size_t stage = ((size_t)PT_HALF * C * esize + (esize == 4 ? 0 : 16) + 127) & ~(size_t)127;
   const size_t aslot = 2 * (size_t)PT_M * 32, dslot = 2 * (size_t)Np * 32;
   const size_t fixed = (size_t)PT_NBAR * 8 + 64;
   PiTcPlan p;
@@ -493,18 +531,25 @@ extern "C" int coda_b200_pi_full_tc_ok(int H, int64_t N, int C, int64_t model_st
   return H >= 1 && N >= 1 && C >= 16 && C <= 128 && C % 4 == 0 && model_stride % 4 == 0;
 }
 
+// the tensor-core and SIMT passes round differently: an fp16 slab is eligible exactly where its fp32 upcast is
+extern "C" int coda_b200_pi_full_tc_ok_f16(int H, int64_t N, int C, int64_t model_stride) {
+  return coda_b200_pi_full_tc_ok(H, N, C, model_stride);
+}
+
 extern "C" size_t coda_b200_pi_full_tc_scratch_bytes(int H, int C) {
   const int Np = (C + 15) / 16 * 16, KC = (C + 15) / 16;
   return (size_t)H * KC * 2 * Np * 16 * 2 + 16;
 }
 
-extern "C" int coda_b200_pi_full_tc(const float* preds, int64_t model_stride, const float* D, int H, int64_t N, int C,
-                                    float* U, void* scratch, uint32_t* flags, coda_stream_t stream) {
+template <typename T>
+static int pi_full_tc(const T* preds, int64_t model_stride, const float* D, int H, int64_t N, int C, float* U,
+                      void* scratch, uint32_t* flags, coda_stream_t stream) {
   CODA_CHECK_ARG(preds && D && U && scratch && flags, "pi_full_tc: null pointer");
   CODA_CHECK_ARG(coda_b200_pi_full_tc_ok(H, N, C, model_stride),
-                 "pi_full_tc: needs 16 <= C <= 128, C %% 4 == 0 and a 16-byte aligned model stride (C=%d)", C);
-  CODA_CHECK_ARG(((uintptr_t)preds & 15) == 0 && ((uintptr_t)U & 15) == 0 && ((uintptr_t)scratch & 15) == 0,
-                 "pi_full_tc: preds, U and scratch must be 16-byte aligned");
+                 "pi_full_tc: needs 16 <= C <= 128, C %% 4 == 0 and a model stride that is a multiple of 4 (C=%d)", C);
+  // fp32: 16-byte aligned copies; fp16: rows 8-byte aligned (the copies take aligned windows)
+  CODA_CHECK_ARG(((uintptr_t)preds & (4 * sizeof(T) - 1)) == 0 && ((uintptr_t)U & 15) == 0 && ((uintptr_t)scratch & 15) == 0,
+                 "pi_full_tc: preds must be %d-byte aligned, U and scratch 16-byte aligned", (int)(4 * sizeof(T)));
   const int Np = (C + 15) / 16 * 16, KC = (C + 15) / 16;
   unsigned char* wb = reinterpret_cast<unsigned char*>(scratch);
   uint32_t* dmax = reinterpret_cast<uint32_t*>(wb + coda_b200_pi_full_tc_scratch_bytes(H, C) - 16);
@@ -513,7 +558,7 @@ extern "C" int coda_b200_pi_full_tc(const float* preds, int64_t model_stride, co
   CODA_LAUNCH_OK("k_pi_w_max");
   k_pi_w_limbs<<<coda_sm_count() * 4, 256, 0, as_stream(stream)>>>(D, H, C, Np, KC, dmax, reinterpret_cast<__half*>(wb));
   CODA_LAUNCH_OK("k_pi_w_limbs");
-  const PiTcPlan plan = pi_tc_plan(C, Np);
+  const PiTcPlan plan = pi_tc_plan(C, Np, sizeof(T));
   CODA_CHECK_ARG(plan.smem <= 227 * 1024, "pi_full_tc: C=%d does not fit shared memory", C);
   PiTcArgs a;
   a.preds = preds; a.ldh = model_stride; a.wb = wb; a.dmax = dmax; a.U = U; a.flags = flags;
@@ -522,9 +567,19 @@ extern "C" int coda_b200_pi_full_tc(const float* preds, int64_t model_stride, co
   // models per drain: the truncating fp32 accumulate of the tensor core loses up to 2^-24 per K = 8 sub-step of the chain
   const char* genv = getenv("CODA_B200_PI_DRAIN");
   a.G = genv ? max(1, min(16, atoi(genv))) : 4;
-  CODA_CUDA_OK(cudaFuncSetAttribute(k_pi_full_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem));
+  CODA_CUDA_OK(cudaFuncSetAttribute(k_pi_full_tc<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem));
   const long long grid = (N + PT_M - 1) / PT_M;
-  k_pi_full_tc<<<(unsigned)grid, PT_THREADS, plan.smem, as_stream(stream)>>>(a);
+  k_pi_full_tc<T><<<(unsigned)grid, PT_THREADS, plan.smem, as_stream(stream)>>>(a);
   CODA_LAUNCH_OK("k_pi_full_tc");
   return CODA_B200_OK;
+}
+
+extern "C" int coda_b200_pi_full_tc(const float* preds, int64_t model_stride, const float* D, int H, int64_t N, int C,
+                                    float* U, void* scratch, uint32_t* flags, coda_stream_t stream) {
+  return pi_full_tc(preds, model_stride, D, H, N, C, U, scratch, flags, stream);
+}
+
+extern "C" int coda_b200_pi_full_tc_f16(const uint16_t* preds, int64_t model_stride, const float* D, int H, int64_t N,
+                                        int C, float* U, void* scratch, uint32_t* flags, coda_stream_t stream) {
+  return pi_full_tc(reinterpret_cast<const __half*>(preds), model_stride, D, H, N, C, U, scratch, flags, stream);
 }

@@ -1,5 +1,5 @@
-// Slab-streaming kernels of the CODA hot path (HBM-bound passes over the (H, N, C) fp32
-// prediction slab) and the Bayesian posterior update.
+// Slab-streaming kernels of the CODA hot path (HBM-bound passes over the (H, N, C) prediction slab, fp32 or fp16,
+// always computed in fp32) and the Bayesian posterior update.
 //
 //   scan_slab          reference coda.py:193-194 (ensemble mean -> pseudo labels),
 //                      coda.py:217-218, 263, 316 (per-model argmax), coda.py:215-219 (unanimity)
@@ -17,7 +17,8 @@
 // ---------------------------------------------------------------------------------------
 // scan_slab: one pass over the slab.  CTA = tile of TN points, all H models.
 // ---------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_scan_slab(const float* __restrict__ preds, long long ldh, int H, long long N, int C,
+template <typename T>
+__global__ void __launch_bounds__(256) k_scan_slab(const T* __restrict__ preds, long long ldh, int H, long long N, int C,
                                                    int TN, uint16_t* __restrict__ hard,
                                                    int32_t* __restrict__ pseudo, uint8_t* __restrict__ disagree,
                                                    float* __restrict__ ens_out, uint32_t* __restrict__ flags) {
@@ -31,14 +32,14 @@ __global__ void __launch_bounds__(256) k_scan_slab(const float* __restrict__ pre
   __syncthreads();
   uint32_t bad = 0;
   for (int h = 0; h < H; ++h) {
-    const float* base = preds + (size_t)h * ldh + (size_t)n0 * C;
+    const T* base = preds + (size_t)h * ldh + (size_t)n0 * C;
     for (int p = warp; p < tn; p += nwarp) {
-      const float* row = base + (size_t)p * C;
+      const T* row = base + (size_t)p * C;
       float* erow = ens + (size_t)p * C;
       float bv = -INFINITY;
       int bi = 0x7fffffff;
       for (int c = lane; c < C; c += 32) {
-        float v = __ldg(row + c);
+        float v = slab_ld(row + c);
         if (!isfinite(v)) bad |= CODA_B200_FLAG_NONFINITE_INPUT;
         if (v < 0.f || v > 1.0001f) bad |= CODA_B200_FLAG_RANGE_INPUT;
         erow[c] += v;
@@ -87,31 +88,29 @@ __global__ void __launch_bounds__(256) k_scan_slab(const float* __restrict__ pre
 // the ensemble sums live in registers.
 #define SS_TN 32
 #define SS_ST 4
-template <int KC>
-__global__ void __launch_bounds__(256) k_scan_slab_tma(const float* __restrict__ preds, long long ldh, int H, long long N, int C,
+template <typename T, int KC>
+__global__ void __launch_bounds__(256) k_scan_slab_tma(const T* __restrict__ preds, long long ldh, int H, long long N, int C,
                                                        uint16_t* __restrict__ hard, int32_t* __restrict__ pseudo,
                                                        uint8_t* __restrict__ disagree, float* __restrict__ ens_out,
                                                        uint32_t* __restrict__ flags) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int tile_floats = SS_TN * C;
-  const size_t buf_bytes = ((size_t)tile_floats * 4 + 127) / 128 * 128;
-  float* bufs = reinterpret_cast<float*>(smem_raw);                                    // [SS_ST][tile]
+  const size_t buf_bytes = ((size_t)tile_floats * sizeof(T) + slab_pad<T>() + 127) / 128 * 128;
+  unsigned char* bufs = smem_raw;                                                      // [SS_ST][tile]
   uint16_t* hard_t = reinterpret_cast<uint16_t*>(smem_raw + SS_ST * buf_bytes);         // [SS_TN][H]
   uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + SS_ST * buf_bytes + (((size_t)SS_TN * H * 2 + 15) / 16) * 16);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long n0 = (long long)blockIdx.x * SS_TN;
   const int tn = (int)min((long long)SS_TN, N - n0);
-  const uint32_t bytes = (uint32_t)tn * C * 4;          // multiple of 16: callers guarantee (tn * C) % 4 == 0
+  const uint32_t bytes = (uint32_t)tn * C * sizeof(T);  // fp32: a multiple of 16, callers guarantee (tn * C) % 4 == 0
   if (threadIdx.x == 0) {
     for (int s = 0; s < SS_ST; ++s) mbar_init(&full[s], 1);
     mbar_fence_init();
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    for (int s = 0; s < SS_ST && s < H; ++s) {
-      mbar_expect_tx(&full[s], bytes);
-      tma_load_1d(reinterpret_cast<unsigned char*>(bufs) + s * buf_bytes, preds + (size_t)s * ldh + (size_t)n0 * C, bytes, &full[s]);
-    }
+    for (int s = 0; s < SS_ST && s < H; ++s)
+      tma_load_slab(bufs + s * buf_bytes, preds + (size_t)s * ldh + (size_t)n0 * C, bytes, &full[s]);
   }
   float ens[4][KC];
 #pragma unroll
@@ -122,7 +121,7 @@ __global__ void __launch_bounds__(256) k_scan_slab_tma(const float* __restrict__
   for (int h = 0; h < H; ++h) {
     const int s = h % SS_ST;
     mbar_wait(&full[s], (h / SS_ST) & 1);
-    const float* buf = reinterpret_cast<const float*>(reinterpret_cast<const unsigned char*>(bufs) + s * buf_bytes);
+    const T* buf = reinterpret_cast<const T*>(bufs + s * buf_bytes + slab_head(preds + (size_t)h * ldh + (size_t)n0 * C));
     float bv[4];
     int bi[4];
 #pragma unroll
@@ -135,7 +134,7 @@ __global__ void __launch_bounds__(256) k_scan_slab_tma(const float* __restrict__
         for (int k = 0; k < KC; ++k) {
           const int c = lane + 32 * k;
           if (c < C) {
-            const float v = buf[p * C + c];
+            const float v = slab_f(buf[p * C + c]);
             if (!isfinite(v)) bad |= CODA_B200_FLAG_NONFINITE_INPUT;
             if (v < 0.f || v > 1.0001f) bad |= CODA_B200_FLAG_RANGE_INPUT;
             ens[r][k] += v;
@@ -161,11 +160,8 @@ __global__ void __launch_bounds__(256) k_scan_slab_tma(const float* __restrict__
       }
     }
     __syncthreads();                                   // everyone is done with buf[s]
-    if (threadIdx.x == 0 && h + SS_ST < H) {
-      mbar_expect_tx(&full[s], bytes);
-      tma_load_1d(reinterpret_cast<unsigned char*>(bufs) + s * buf_bytes, preds + (size_t)(h + SS_ST) * ldh + (size_t)n0 * C, bytes,
-                  &full[s]);
-    }
+    if (threadIdx.x == 0 && h + SS_ST < H)
+      tma_load_slab(bufs + s * buf_bytes, preds + (size_t)(h + SS_ST) * ldh + (size_t)n0 * C, bytes, &full[s]);
   }
   {
     uint16_t* dst = hard + (size_t)n0 * H;
@@ -201,24 +197,26 @@ __global__ void __launch_bounds__(256) k_scan_slab_tma(const float* __restrict__
   if (bad) atomicOr(flags, bad);
 }
 
-extern "C" int coda_b200_scan_slab(const float* preds, int64_t model_stride, int H, int64_t N, int C, uint16_t* hard,
-                                   int32_t* pseudo, uint8_t* disagree, float* ens_out, uint32_t* flags,
-                                   coda_stream_t stream) {
+template <typename T>
+static int scan_slab(const T* preds, int64_t model_stride, int H, int64_t N, int C, uint16_t* hard, int32_t* pseudo,
+                     uint8_t* disagree, float* ens_out, uint32_t* flags, coda_stream_t stream) {
   CODA_CHECK_ARG(preds && hard && pseudo && disagree && flags, "scan_slab: null pointer");
   CODA_CHECK_ARG(model_stride >= (int64_t)N * C, "scan_slab: model_stride %lld < N*C", (long long)model_stride);
   const long long ldh = model_stride;
   CODA_CHECK_ARG(H >= 1 && C >= 2 && C <= 65535 && N >= 1, "scan_slab: bad dims H=%d N=%lld C=%d", H, (long long)N, C);
+  // bulk-TMA path when every copy of an fp32 slab is 16-byte aligned.  A 16-bit slab takes it for the same shapes and
+  // views (element offsets that are multiples of 4: an 8-byte aligned pointer) and copies aligned windows.
   if (C <= 128 && ldh % 4 == 0 && ((long long)SS_TN * C) % 4 == 0 && ((N % SS_TN) * C) % 4 == 0 &&
-      (reinterpret_cast<uintptr_t>(preds) & 15) == 0) {
-    const size_t buf_bytes = ((size_t)SS_TN * C * 4 + 127) / 128 * 128;
+      (reinterpret_cast<uintptr_t>(preds) & (4 * sizeof(T) - 1)) == 0) {
+    const size_t buf_bytes = ((size_t)SS_TN * C * sizeof(T) + slab_pad<T>() + 127) / 128 * 128;
     const size_t smem = SS_ST * buf_bytes + (((size_t)SS_TN * H * 2 + 15) / 16) * 16 + SS_ST * 8;
     if (smem <= 200 * 1024) {
       const long long grid = (N + SS_TN - 1) / SS_TN;
       cudaStream_t st = as_stream(stream);
 #define LAUNCH_SS(KC)                                                                                             \
   do {                                                                                                            \
-    CODA_CUDA_OK(cudaFuncSetAttribute(k_scan_slab_tma<KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    k_scan_slab_tma<KC><<<(unsigned)grid, 256, smem, st>>>(preds, ldh, H, N, C, hard, pseudo, disagree, ens_out, flags); \
+    CODA_CUDA_OK(cudaFuncSetAttribute(k_scan_slab_tma<T, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    k_scan_slab_tma<T, KC><<<(unsigned)grid, 256, smem, st>>>(preds, ldh, H, N, C, hard, pseudo, disagree, ens_out, flags); \
   } while (0)
       if (C <= 32) LAUNCH_SS(1);
       else if (C <= 64) LAUNCH_SS(2);
@@ -237,11 +235,24 @@ extern "C" int coda_b200_scan_slab(const float* preds, int64_t model_stride, int
     TN >>= 1;
   }
   CODA_CHECK_ARG(need <= 200 * 1024, "scan_slab: H=%d C=%d does not fit shared memory", H, C);
-  CODA_CUDA_OK(cudaFuncSetAttribute(k_scan_slab, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
+  CODA_CUDA_OK(cudaFuncSetAttribute(k_scan_slab<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
   long long grid = (N + TN - 1) / TN;
-  k_scan_slab<<<(unsigned)grid, 256, need, as_stream(stream)>>>(preds, ldh, H, N, C, TN, hard, pseudo, disagree, ens_out, flags);
+  k_scan_slab<T><<<(unsigned)grid, 256, need, as_stream(stream)>>>(preds, ldh, H, N, C, TN, hard, pseudo, disagree, ens_out, flags);
   CODA_LAUNCH_OK("k_scan_slab");
   return CODA_B200_OK;
+}
+
+extern "C" int coda_b200_scan_slab(const float* preds, int64_t model_stride, int H, int64_t N, int C, uint16_t* hard,
+                                   int32_t* pseudo, uint8_t* disagree, float* ens_out, uint32_t* flags,
+                                   coda_stream_t stream) {
+  return scan_slab(preds, model_stride, H, N, C, hard, pseudo, disagree, ens_out, flags, stream);
+}
+
+extern "C" int coda_b200_scan_slab_f16(const uint16_t* preds, int64_t model_stride, int H, int64_t N, int C,
+                                       uint16_t* hard, int32_t* pseudo, uint8_t* disagree, float* ens_out,
+                                       uint32_t* flags, coda_stream_t stream) {
+  return scan_slab(reinterpret_cast<const __half*>(preds), model_stride, H, N, C, hard, pseudo, disagree, ens_out, flags,
+                   stream);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -249,7 +260,8 @@ extern "C" int coda_b200_scan_slab(const float* preds, int64_t model_stride, int
 // result does not depend on summation order or on how N is sharded across GPUs.
 // grid = (chunks, H).  Shared-memory table when C*C*8 fits, global atomics otherwise.
 // ---------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_confusion_accum(const float* __restrict__ preds, long long ldh,
+template <typename T>
+__global__ void __launch_bounds__(256) k_confusion_accum(const T* __restrict__ preds, long long ldh,
                                                          const int32_t* __restrict__ pseudo, int H, long long N,
                                                          int C, float fxs, long long chunk, int use_smem,
                                                          unsigned long long* __restrict__ conf_fx) {
@@ -267,10 +279,10 @@ __global__ void __launch_bounds__(256) k_confusion_accum(const float* __restrict
   unsigned long long* dst_tab = use_smem ? tab : gtab;
   for (long long n = n_lo + warp; n < n_hi; n += nwarp) {
     const int y = pseudo[n];
-    const float* row = preds + (size_t)h * ldh + (size_t)n * C;
+    const T* row = preds + (size_t)h * ldh + (size_t)n * C;
     unsigned long long* dst = dst_tab + (size_t)y * C;
     for (int j = lane; j < C; j += 32) {
-      long long v = to_fx(__ldg(row + j), fxs);
+      long long v = to_fx(slab_ld(row + j), fxs);
       if (v != 0) atomicAdd(dst + j, (unsigned long long)v);
     }
   }
@@ -287,8 +299,8 @@ __global__ void __launch_bounds__(256) k_confusion_accum(const float* __restrict
 // keeps the int64 column sums of the current class in registers (lane <-> column j) and flushes them with a
 // handful of global atomics when the class changes -- no shared-memory atomics on the slab-sized stream.
 #define CS_RUN 256
-template <int KC>
-__global__ void __launch_bounds__(256) k_confusion_sorted(const float* __restrict__ preds, long long ldh,
+template <typename T, int KC>
+__global__ void __launch_bounds__(256) k_confusion_sorted(const T* __restrict__ preds, long long ldh,
                                                           const int32_t* __restrict__ pseudo,
                                                           const int32_t* __restrict__ order, int H, long long N, int C,
                                                           float fxs, unsigned long long* __restrict__ conf_fx) {
@@ -297,7 +309,7 @@ __global__ void __launch_bounds__(256) k_confusion_sorted(const float* __restric
   const long long i0 = ((long long)blockIdx.x * 8 + warp) * CS_RUN;
   const long long i1 = min(N, i0 + CS_RUN);
   if (i0 >= N) return;
-  const float* slab = preds + (size_t)h * ldh;
+  const T* slab = preds + (size_t)h * ldh;
   unsigned long long* tab = conf_fx + (size_t)h * C * C;
   long long acc[KC];
 #pragma unroll
@@ -323,11 +335,11 @@ __global__ void __launch_bounds__(256) k_confusion_sorted(const float* __restric
     }
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
-      const float* row = slab + (size_t)n[q] * C;
+      const T* row = slab + (size_t)n[q] * C;
 #pragma unroll
       for (int k = 0; k < KC; ++k) {
         const int j = lane + 32 * k;
-        v[q][k] = j < C ? __ldg(row + j) : 0.f;
+        v[q][k] = j < C ? slab_ld(row + j) : 0.f;
       }
     }
 #pragma unroll
@@ -344,9 +356,9 @@ __global__ void __launch_bounds__(256) k_confusion_sorted(const float* __restric
   flush();
 }
 
-extern "C" int coda_b200_confusion_sorted(const float* preds, int64_t model_stride, const int32_t* pseudo,
-                                          const int32_t* order, int H, int64_t N, int C, int fx_shift,
-                                          int64_t* conf_fx, coda_stream_t stream) {
+template <typename T>
+static int confusion_sorted(const T* preds, int64_t model_stride, const int32_t* pseudo, const int32_t* order, int H,
+                            int64_t N, int C, int fx_shift, int64_t* conf_fx, coda_stream_t stream) {
   const long long ldh = model_stride;
   CODA_CHECK_ARG(preds && pseudo && order && conf_fx, "confusion_sorted: null pointer");
   CODA_CHECK_ARG(fx_shift >= 8 && fx_shift <= 46, "confusion_sorted: bad fx_shift %d", fx_shift);
@@ -356,29 +368,53 @@ extern "C" int coda_b200_confusion_sorted(const float* preds, int64_t model_stri
   const float fxs = exp2f((float)fx_shift);
   unsigned long long* out = reinterpret_cast<unsigned long long*>(conf_fx);
   cudaStream_t st = as_stream(stream);
-  if (C <= 32) k_confusion_sorted<1><<<grid, 256, 0, st>>>(preds, ldh, pseudo, order, H, N, C, fxs, out);
-  else if (C <= 64) k_confusion_sorted<2><<<grid, 256, 0, st>>>(preds, ldh, pseudo, order, H, N, C, fxs, out);
-  else if (C <= 96) k_confusion_sorted<3><<<grid, 256, 0, st>>>(preds, ldh, pseudo, order, H, N, C, fxs, out);
-  else k_confusion_sorted<4><<<grid, 256, 0, st>>>(preds, ldh, pseudo, order, H, N, C, fxs, out);
+  if (C <= 32) k_confusion_sorted<T, 1><<<grid, 256, 0, st>>>(preds, ldh, pseudo, order, H, N, C, fxs, out);
+  else if (C <= 64) k_confusion_sorted<T, 2><<<grid, 256, 0, st>>>(preds, ldh, pseudo, order, H, N, C, fxs, out);
+  else if (C <= 96) k_confusion_sorted<T, 3><<<grid, 256, 0, st>>>(preds, ldh, pseudo, order, H, N, C, fxs, out);
+  else k_confusion_sorted<T, 4><<<grid, 256, 0, st>>>(preds, ldh, pseudo, order, H, N, C, fxs, out);
   CODA_LAUNCH_OK("k_confusion_sorted");
   return CODA_B200_OK;
 }
 
-extern "C" int coda_b200_confusion_accum(const float* preds, int64_t model_stride, const int32_t* pseudo, int H,
-                                         int64_t N, int C, int fx_shift, int64_t* conf_fx, coda_stream_t stream) {
+extern "C" int coda_b200_confusion_sorted(const float* preds, int64_t model_stride, const int32_t* pseudo,
+                                          const int32_t* order, int H, int64_t N, int C, int fx_shift,
+                                          int64_t* conf_fx, coda_stream_t stream) {
+  return confusion_sorted(preds, model_stride, pseudo, order, H, N, C, fx_shift, conf_fx, stream);
+}
+
+extern "C" int coda_b200_confusion_sorted_f16(const uint16_t* preds, int64_t model_stride, const int32_t* pseudo,
+                                              const int32_t* order, int H, int64_t N, int C, int fx_shift,
+                                              int64_t* conf_fx, coda_stream_t stream) {
+  return confusion_sorted(reinterpret_cast<const __half*>(preds), model_stride, pseudo, order, H, N, C, fx_shift, conf_fx,
+                          stream);
+}
+
+template <typename T>
+static int confusion_accum(const T* preds, int64_t model_stride, const int32_t* pseudo, int H, int64_t N, int C,
+                           int fx_shift, int64_t* conf_fx, coda_stream_t stream) {
   CODA_CHECK_ARG(preds && pseudo && conf_fx, "confusion_accum: null pointer");
   CODA_CHECK_ARG(fx_shift >= 8 && fx_shift <= 46, "confusion_accum: bad fx_shift %d", fx_shift);
   size_t tab = (size_t)C * C * 8;
   int use_smem = tab <= 160 * 1024;
   size_t smem = use_smem ? tab : 0;
-  if (use_smem) CODA_CUDA_OK(cudaFuncSetAttribute(k_confusion_accum, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (use_smem) CODA_CUDA_OK(cudaFuncSetAttribute(k_confusion_accum<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   long long chunk = 8192;
   long long chunks = (N + chunk - 1) / chunk;
   dim3 grid((unsigned)chunks, (unsigned)H);
-  k_confusion_accum<<<grid, 256, smem, as_stream(stream)>>>(preds, (long long)model_stride, pseudo, H, N, C, exp2f((float)fx_shift), chunk, use_smem,
+  k_confusion_accum<T><<<grid, 256, smem, as_stream(stream)>>>(preds, (long long)model_stride, pseudo, H, N, C, exp2f((float)fx_shift), chunk, use_smem,
                                                            reinterpret_cast<unsigned long long*>(conf_fx));
   CODA_LAUNCH_OK("k_confusion_accum");
   return CODA_B200_OK;
+}
+
+extern "C" int coda_b200_confusion_accum(const float* preds, int64_t model_stride, const int32_t* pseudo, int H,
+                                         int64_t N, int C, int fx_shift, int64_t* conf_fx, coda_stream_t stream) {
+  return confusion_accum(preds, model_stride, pseudo, H, N, C, fx_shift, conf_fx, stream);
+}
+
+extern "C" int coda_b200_confusion_accum_f16(const uint16_t* preds, int64_t model_stride, const int32_t* pseudo, int H,
+                                             int64_t N, int C, int fx_shift, int64_t* conf_fx, coda_stream_t stream) {
+  return confusion_accum(reinterpret_cast<const __half*>(preds), model_stride, pseudo, H, N, C, fx_shift, conf_fx, stream);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -428,7 +464,8 @@ extern "C" int coda_b200_init_dirichlets(const int64_t* conf_fx, const int64_t* 
 #define PF_TN 64
 #define PF_TC 128
 #define PF_SK 32
-__global__ void __launch_bounds__(256) k_pi_full(const float* __restrict__ preds, long long ldh,
+template <typename T>
+__global__ void __launch_bounds__(256) k_pi_full(const T* __restrict__ preds, long long ldh,
                                                  const float* __restrict__ D, int H, long long N, int C,
                                                  float* __restrict__ U) {
   __shared__ float As[PF_TN][PF_SK + 1];
@@ -443,7 +480,7 @@ __global__ void __launch_bounds__(256) k_pi_full(const float* __restrict__ preds
 #pragma unroll
       for (int k = 0; k < 8; ++k) acc[i][k] = 0.f;
     for (int h = 0; h < H; ++h) {
-      const float* Ah = preds + (size_t)h * ldh;
+      const T* Ah = preds + (size_t)h * ldh;
       const float* Dh = D + ((size_t)h * C) * C;
       for (int s0 = 0; s0 < C; s0 += PF_SK) {
         __syncthreads();
@@ -451,7 +488,7 @@ __global__ void __launch_bounds__(256) k_pi_full(const float* __restrict__ preds
           int r = e >> 5, col = e & 31;
           long long n = n0 + r;
           int s = s0 + col;
-          As[r][col] = (n < N && s < C) ? __ldg(Ah + (size_t)n * C + s) : 0.f;
+          As[r][col] = (n < N && s < C) ? slab_ld(Ah + (size_t)n * C + s) : 0.f;
         }
         for (int e = tid; e < PF_TC * PF_SK; e += 256) {
           int r = e >> 5, col = e & 31;
@@ -486,13 +523,24 @@ __global__ void __launch_bounds__(256) k_pi_full(const float* __restrict__ preds
   }
 }
 
-extern "C" int coda_b200_pi_full(const float* preds, int64_t model_stride, const float* D, int H, int64_t N, int C,
-                                 float* U, coda_stream_t stream) {
+template <typename T>
+static int pi_full(const T* preds, int64_t model_stride, const float* D, int H, int64_t N, int C, float* U,
+                   coda_stream_t stream) {
   CODA_CHECK_ARG(preds && D && U, "pi_full: null pointer");
   long long grid = (N + PF_TN - 1) / PF_TN;
-  k_pi_full<<<(unsigned)grid, 256, 0, as_stream(stream)>>>(preds, (long long)model_stride, D, H, N, C, U);
+  k_pi_full<T><<<(unsigned)grid, 256, 0, as_stream(stream)>>>(preds, (long long)model_stride, D, H, N, C, U);
   CODA_LAUNCH_OK("k_pi_full");
   return CODA_B200_OK;
+}
+
+extern "C" int coda_b200_pi_full(const float* preds, int64_t model_stride, const float* D, int H, int64_t N, int C,
+                                 float* U, coda_stream_t stream) {
+  return pi_full(preds, model_stride, D, H, N, C, U, stream);
+}
+
+extern "C" int coda_b200_pi_full_f16(const uint16_t* preds, int64_t model_stride, const float* D, int H, int64_t N, int C,
+                                     float* U, coda_stream_t stream) {
+  return pi_full(reinterpret_cast<const __half*>(preds), model_stride, D, H, N, C, U, stream);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -574,20 +622,21 @@ extern "C" int coda_b200_pi_reduce(float* U, int64_t N, int C, int fx_shift, flo
 // layout that costs a 64-byte DRAM fetch each, from the shadow it is a coalesced 4-byte read.
 // grid = (ceil(N/32), ceil(C/32), S), block = (32, 8)
 // ---------------------------------------------------------------------------------------
-__global__ void k_shadow_transpose(const float* __restrict__ preds, long long ldh, long long N, int C,
-                                   const int32_t* __restrict__ model_of_slot, long long cs, float* __restrict__ T) {
-  __shared__ float tile[32][33];
+template <typename E>
+__global__ void k_shadow_transpose(const E* __restrict__ preds, long long ldh, long long N, int C,
+                                   const int32_t* __restrict__ model_of_slot, long long cs, E* __restrict__ T) {
+  __shared__ E tile[32][33];
   const int s = blockIdx.z, h = model_of_slot[s];
   const long long n0 = (long long)blockIdx.x * 32;
   const int c0 = blockIdx.y * 32;
-  const float* src = preds + (size_t)h * ldh;
+  const E* src = preds + (size_t)h * ldh;
   for (int r = threadIdx.y; r < 32; r += 8) {
     const long long n = n0 + r;
     const int c = c0 + threadIdx.x;
-    tile[r][threadIdx.x] = (n < N && c < C) ? __ldg(src + (size_t)n * C + c) : 0.f;
+    tile[r][threadIdx.x] = (n < N && c < C) ? __ldg(src + (size_t)n * C + c) : E(0.f);
   }
   __syncthreads();
-  float* dst = T + (size_t)s * C * cs;
+  E* dst = T + (size_t)s * C * cs;
   for (int r = threadIdx.y; r < 32; r += 8) {
     const int c = c0 + r;
     const long long n = n0 + threadIdx.x;
@@ -595,17 +644,32 @@ __global__ void k_shadow_transpose(const float* __restrict__ preds, long long ld
   }
 }
 
-extern "C" int coda_b200_shadow_build(const float* preds, int64_t model_stride, int H, int64_t N, int C,
-                                      const int32_t* model_of_slot, int S, int64_t col_stride, float* T,
-                                      coda_stream_t stream) {
+template <typename E>
+static int shadow_build(const E* preds, int64_t model_stride, int H, int64_t N, int C, const int32_t* model_of_slot, int S,
+                        int64_t col_stride, E* T, coda_stream_t stream) {
   CODA_CHECK_ARG(preds && model_of_slot && T && S >= 1 && S <= H && col_stride >= N, "shadow_build: bad arguments");
+  CODA_CHECK_ARG(sizeof(E) == 4 || col_stride % 8 == 0, "shadow_build: col_stride %lld leaves fp16 columns unaligned",
+                 (long long)col_stride);
   long long gx = (N + 31) / 32;
   CODA_CHECK_ARG(gx <= 0x7fffffffLL && S <= 65535, "shadow_build: grid too large");
   dim3 grid((unsigned)gx, (unsigned)((C + 31) / 32), (unsigned)S), block(32, 8);
-  k_shadow_transpose<<<grid, block, 0, as_stream(stream)>>>(preds, (long long)model_stride, N, C, model_of_slot,
-                                                            (long long)col_stride, T);
+  k_shadow_transpose<E><<<grid, block, 0, as_stream(stream)>>>(preds, (long long)model_stride, N, C, model_of_slot,
+                                                               (long long)col_stride, T);
   CODA_LAUNCH_OK("k_shadow_transpose");
   return CODA_B200_OK;
+}
+
+extern "C" int coda_b200_shadow_build(const float* preds, int64_t model_stride, int H, int64_t N, int C,
+                                      const int32_t* model_of_slot, int S, int64_t col_stride, float* T,
+                                      coda_stream_t stream) {
+  return shadow_build(preds, model_stride, H, N, C, model_of_slot, S, col_stride, T, stream);
+}
+
+extern "C" int coda_b200_shadow_build_f16(const uint16_t* preds, int64_t model_stride, int H, int64_t N, int C,
+                                          const int32_t* model_of_slot, int S, int64_t col_stride, uint16_t* T,
+                                          coda_stream_t stream) {
+  return shadow_build(reinterpret_cast<const __half*>(preds), model_stride, H, N, C, model_of_slot, S, col_stride,
+                      reinterpret_cast<__half*>(T), stream);
 }
 
 // register variant of row_accumulate for C <= 32 * KC: NR rows per call (all loads issued before the first
@@ -659,8 +723,8 @@ __constant__ R1Term c_terms_bank[R1_CONST_TERMS];
 #define R1_TN 256
 // GU: gathers in flight per lane, NR: U rows in flight per warp (more of both = more bytes in flight per SM at
 // the price of registers / resident warps)
-template <int KC, int GU = 16, int NR = 4, bool CONST_TERMS = false>
-__global__ void __launch_bounds__(256, (GU > 16 ? 3 : 4)) k_pi_rank1(const float* __restrict__ preds, const float* __restrict__ E,
+template <typename T, int KC, int GU = 16, int NR = 4, bool CONST_TERMS = false>
+__global__ void __launch_bounds__(256, (GU > 16 ? 3 : 4)) k_pi_rank1(const T* __restrict__ preds, const float* __restrict__ E,
                                                   long long N, int C, const long long* __restrict__ sel,
                                                   const int32_t* __restrict__ hdr, const R1Term* __restrict__ gterms,
                                                   int const_base, float lr, float fxs,
@@ -694,11 +758,11 @@ __global__ void __launch_bounds__(256, (GU > 16 ? 3 : 4)) k_pi_rank1(const float
       for (; k + GU <= nt; k += GU) {
         float v[GU];
 #pragma unroll
-        for (int q = 0; q < GU; ++q) v[q] = __ldg(preds + c_terms[k + q].off + n * c_terms[k + q].str);
+        for (int q = 0; q < GU; ++q) v[q] = slab_ld(preds + c_terms[k + q].off + n * c_terms[k + q].str);
 #pragma unroll
         for (int q = 0; q < GU; ++q) d = fmaf(c_terms[k + q].sg, v[q], d);
       }
-      for (; k < nt; ++k) d = fmaf(c_terms[k].sg, __ldg(preds + c_terms[k].off + n * c_terms[k].str), d);
+      for (; k < nt; ++k) d = fmaf(c_terms[k].sg, slab_ld(preds + c_terms[k].off + n * c_terms[k].str), d);
     }
     const float dl = lr * d;
     const int rows = (int)min(32LL, N - n0);
@@ -1017,10 +1081,10 @@ static int r1x_tile_rows(int C) {     // rows per tile: U tile <= ~104 KB, multi
   return tr;
 }
 
-extern "C" int coda_b200_pi_rank1(const float* preds, const float* ens, int H, int64_t N, int C, const int64_t* sel,
-                                  double lr, int fx_shift, const int32_t* terms /*[2 + 8H]*/, float* U,
-                                  int64_t* pisum_fx, uint32_t* flags, int ctas_per_sm, int const_slot,
-                                  coda_stream_t stream) {
+template <typename T>
+static int pi_rank1(const T* preds, const float* ens, int H, int64_t N, int C, const int64_t* sel, double lr,
+                    int fx_shift, const int32_t* terms /*[2 + 8H]*/, float* U, int64_t* pisum_fx, uint32_t* flags,
+                    int ctas_per_sm, int const_slot, coda_stream_t stream) {
   CODA_CHECK_ARG(preds && sel && terms && U && pisum_fx && flags, "pi_rank1: null pointer");
   CODA_CHECK_ARG(2 * H <= R1_MAXT, "pi_rank1: H=%d too large", H);
   CODA_CHECK_ARG((reinterpret_cast<uintptr_t>(terms) & 7) == 0, "pi_rank1: terms must be 8-byte aligned");
@@ -1036,8 +1100,11 @@ extern "C" int coda_b200_pi_rank1(const float* preds, const float* ens, int H, i
   const bool want_v1 = !(r1env && r1env[0] == 'v' && r1env[1] == '4');
   const bool want_deep = r1env && r1env[0] == 'v' && r1env[1] == '1' && r1env[2] == 'd';   // "v1d": 32 gathers / 8 rows in flight
   const bool no_tma = !want_tma;
+  // the "tma" and "v4" variants read the slab as fp32 words (bulk copies of shadow columns, float4 runs): fp32 only
+  CODA_CHECK_ARG(sizeof(T) == 4 || (!want_tma && want_v1),
+                 "pi_rank1: CODA_B200_R1=%s is not available for a 16-bit slab (use v1 or v1d)", r1env ? r1env : "");
   const int TR = C <= 128 ? r1x_tile_rows(C) : 0;
-  if (!no_tma && TR >= 32 && (reinterpret_cast<uintptr_t>(U) & 15) == 0) {
+  if constexpr (sizeof(T) == 4) if (!no_tma && TR >= 32 && (reinterpret_cast<uintptr_t>(U) & 15) == 0) {
     const size_t u_bytes = ((size_t)TR * C * 4 + 127) & ~(size_t)127;
     const size_t smem_x = u_bytes + (size_t)R1X_ST * R1X_TB * TR * 4 + (size_t)2 * H * sizeof(R1Term) + (size_t)8 * C * 8 +
                           (size_t)2 * H * 4 + 8 + (2 + 2 * R1X_ST) * 8;
@@ -1063,7 +1130,7 @@ extern "C" int coda_b200_pi_rank1(const float* preds, const float* ens, int H, i
   }
   size_t smem = (size_t)8 * C * 8 + (size_t)2 * H * sizeof(R1Term);
   CODA_CHECK_ARG(smem <= 200 * 1024, "pi_rank1: C=%d too large", C);
-  if (!want_v1 && C <= 128) {
+  if constexpr (sizeof(T) == 4) if (!want_v1 && C <= 128) {
     long long want4 = (N + 8 * R1V_WI - 1) / (8 * R1V_WI);
     int cps = (ctas_per_sm < 1 || ctas_per_sm > 8) ? 8 : ctas_per_sm;
     int grid4 = (int)min(want4, (long long)coda_sm_count() * cps);
@@ -1094,20 +1161,20 @@ extern "C" int coda_b200_pi_rank1(const float* preds, const float* ens, int H, i
 #define LAUNCH_R1(KC)                                                                                          \
   do {                                                                                                         \
     if (use_const) {                                                                                           \
-      CODA_CUDA_OK(cudaFuncSetAttribute(k_pi_rank1<KC, 16, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-      k_pi_rank1<KC, 16, 4, true><<<grid, 256, smem, st>>>(preds, ens, N, C, reinterpret_cast<const long long*>(sel), hdr, \
+      CODA_CUDA_OK(cudaFuncSetAttribute(k_pi_rank1<T, KC, 16, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+      k_pi_rank1<T, KC, 16, 4, true><<<grid, 256, smem, st>>>(preds, ens, N, C, reinterpret_cast<const long long*>(sel), hdr, \
                                             tlist, const_base, (float)lr, exp2f((float)fx_shift), U,           \
                                             reinterpret_cast<unsigned long long*>(pisum_fx), flags);           \
       break;                                                                                                   \
     }                                                                                                          \
-    CODA_CUDA_OK(cudaFuncSetAttribute(k_pi_rank1<KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    k_pi_rank1<KC><<<grid, 256, smem, st>>>(preds, ens, N, C, reinterpret_cast<const long long*>(sel), hdr,    \
+    CODA_CUDA_OK(cudaFuncSetAttribute(k_pi_rank1<T, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    k_pi_rank1<T, KC><<<grid, 256, smem, st>>>(preds, ens, N, C, reinterpret_cast<const long long*>(sel), hdr,    \
                                             tlist, 0, (float)lr, exp2f((float)fx_shift), U,                    \
                                             reinterpret_cast<unsigned long long*>(pisum_fx), flags);           \
   } while (0)
   if (want_deep && C > 64 && C <= 128) {
-    CODA_CUDA_OK(cudaFuncSetAttribute(k_pi_rank1<4, 32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_pi_rank1<4, 32, 8><<<grid, 256, smem, st>>>(preds, ens, N, C, reinterpret_cast<const long long*>(sel), hdr, tlist, 0,
+    CODA_CUDA_OK(cudaFuncSetAttribute(k_pi_rank1<T, 4, 32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_pi_rank1<T, 4, 32, 8><<<grid, 256, smem, st>>>(preds, ens, N, C, reinterpret_cast<const long long*>(sel), hdr, tlist, 0,
                                                   (float)lr, exp2f((float)fx_shift), U,
                                                   reinterpret_cast<unsigned long long*>(pisum_fx), flags);
     CODA_LAUNCH_OK("k_pi_rank1<deep>");
@@ -1120,4 +1187,19 @@ extern "C" int coda_b200_pi_rank1(const float* preds, const float* ens, int H, i
 #undef LAUNCH_R1
   CODA_LAUNCH_OK("k_pi_rank1");
   return CODA_B200_OK;
+}
+
+extern "C" int coda_b200_pi_rank1(const float* preds, const float* ens, int H, int64_t N, int C, const int64_t* sel,
+                                  double lr, int fx_shift, const int32_t* terms /*[2 + 8H]*/, float* U,
+                                  int64_t* pisum_fx, uint32_t* flags, int ctas_per_sm, int const_slot,
+                                  coda_stream_t stream) {
+  return pi_rank1(preds, ens, H, N, C, sel, lr, fx_shift, terms, U, pisum_fx, flags, ctas_per_sm, const_slot, stream);
+}
+
+extern "C" int coda_b200_pi_rank1_f16(const uint16_t* preds, const float* ens, int H, int64_t N, int C,
+                                      const int64_t* sel, double lr, int fx_shift, const int32_t* terms, float* U,
+                                      int64_t* pisum_fx, uint32_t* flags, int ctas_per_sm, int const_slot,
+                                      coda_stream_t stream) {
+  return pi_rank1(reinterpret_cast<const __half*>(preds), ens, H, N, C, sel, lr, fx_shift, terms, U, pisum_fx, flags,
+                  ctas_per_sm, const_slot, stream);
 }

@@ -8,13 +8,28 @@ import torch
 from .synth import shard_range, synth, synth_compact
 
 
+def keep_fp16_default() -> bool:
+    """``CODA_B200_KEEP_FP16=1`` makes ``keep_fp16=True`` the loaders' default (for drivers that build ``Dataset`` with
+    the reference's two arguments, e.g. main.py through the ``coda`` shim)."""
+    return os.environ.get("CODA_B200_KEEP_FP16", "0") == "1"
+
+
+def _slab_dtype(t, keep_fp16):
+    """fp16 scores stay fp16 with ``keep_fp16`` (the kernels read them as they are and compute in fp32: the run is
+    bit-identical to one on the upcast slab, with half the memory); everything else is upcast to fp32 as the reference
+    loader does (coda/datasets.py:14).  Nothing is ever rounded."""
+    return torch.float16 if (keep_fp16 and t.dtype == torch.float16) else torch.float32
+
+
 class Dataset:
     """(H, N, C) post-softmax scores from ``filepath`` (+ optional ``*_labels.pt``), forced to fp32
-    (coda/datasets.py:12-23)."""
+    (coda/datasets.py:12-23) unless ``keep_fp16`` keeps an fp16 file fp16 (default: ``CODA_B200_KEEP_FP16``)."""
 
-    def __init__(self, filepath, device):
+    def __init__(self, filepath, device, keep_fp16=None):
         self.device = device
-        self.preds = torch.load(filepath, map_location=device).float().contiguous()
+        keep = keep_fp16_default() if keep_fp16 is None else bool(keep_fp16)
+        preds = torch.load(filepath, map_location=device)
+        self.preds = preds.to(_slab_dtype(preds, keep)).contiguous()
         print("Loaded preds of shape", self.preds.shape)
         self.labels = None
         label_p = filepath.replace(".pt", "_labels.pt")
@@ -37,15 +52,17 @@ class TensorDataset:
 class ShardedFileDataset(TensorDataset):
     """This rank's contiguous N-range of an (H, N, C) ``.pt`` slab, read through ``torch.load(mmap=True)`` so that
     no rank ever materialises the whole tensor (the reference loader, coda/datasets.py:14, loads all of it onto
-    one device).  Labels (``*_labels.pt``, N int64) are small and replicated."""
+    one device).  Labels (``*_labels.pt``, N int64) are small and replicated.  ``keep_fp16`` as for ``Dataset``."""
 
-    def __init__(self, filepath, device, rank=0, world=1):
+    def __init__(self, filepath, device, rank=0, world=1, keep_fp16=None):
+        keep = keep_fp16_default() if keep_fp16 is None else bool(keep_fp16)
         full = torch.load(filepath, map_location="cpu", mmap=True, weights_only=True)
         if full.dim() != 3:
             raise ValueError(f"{filepath}: expected an (H, N, C) tensor, got shape {tuple(full.shape)}")
         n = int(full.shape[1])
         lo, hi = shard_range(n, rank, world)
-        preds = full[:, lo:hi].float().contiguous().to(device)     # avoid fp16 precision errors (coda/datasets.py:14)
+        # avoid fp16 precision errors (coda/datasets.py:14): the kernels compute in fp32 whatever the storage type
+        preds = full[:, lo:hi].to(_slab_dtype(full, keep)).contiguous().to(device)
         labels = None
         label_p = filepath.replace(".pt", "_labels.pt")
         if os.path.exists(label_p):

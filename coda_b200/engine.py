@@ -60,6 +60,14 @@ def _ptr(t):
     return t.data_ptr() if t is not None else None
 
 
+def shadow_slots(spare_bytes, H, N, C, esize):
+    """(model slots, column stride in elements) of a class-major shadow of ``esize``-byte elements in ``spare_bytes``:
+    every (slot, class) column starts 16-byte aligned, so an fp16 shadow fits twice the models of an fp32 one."""
+    per16 = 16 // esize
+    cs = (N + per16 - 1) // per16 * per16
+    return int(min(H, max(0, spare_bytes // (cs * C * esize)))), cs
+
+
 class Engine:
     rep_words = REP_WORDS
 
@@ -81,13 +89,17 @@ class Engine:
                 raise NotImplementedError("coda_b200: mode='recompute_all' is not offered for a compact slab")
             self.K = self.compact.K
         else:
-            if preds.dtype != torch.float32 or preds.dim() != 3:
-                raise TypeError("coda_b200: preds must be a float32 (H, N, C) tensor (coda/datasets.py:14)")
+            if preds.dtype not in (torch.float32, torch.float16) or preds.dim() != 3:
+                raise TypeError("coda_b200: preds must be a float32 or float16 (H, N, C) tensor (coda/datasets.py:14)")
             if not (preds.stride(2) == 1 and preds.stride(1) == Cc and (H == 1 or preds.stride(0) >= N * Cc)):
                 raise ValueError("coda_b200: preds must be (H, N, C) with contiguous items (an N-range view of a "
                                  "contiguous slab is fine)")
         self.lib = nat.load()
         self.preds = preds
+        # an fp16 slab stays fp16 on the device: the `_f16` entry points convert on load and give the bits of the fp32
+        # run on preds.float(); every buffer derived from it (ensemble sums, U, D, ...) is fp32 as before
+        self.f16 = self.compact is None and preds.dtype == torch.float16
+        self.esize = 2 if self.f16 else 4                     # bytes per slab element
         self.dev = preds.device
         with torch.cuda.device(self.dev):
             nat.require_device()
@@ -253,7 +265,7 @@ class Engine:
         st.hard, st.labeled, st.D, st.jvec, st.sel = _ptr(self.hard), _ptr(self.labeled), _ptr(self.D), _ptr(self.jvec), _ptr(self.sel)
         st.terms = _ptr(self.terms)
         st.slot_of_model = _ptr(self.slot_of_model)
-        st.shadow_off = ((self.shadow.data_ptr() - self._slab_ptr()) // 4) if self.shadow is not None else 0
+        st.shadow_off = ((self.shadow.data_ptr() - self._slab_ptr()) // self.esize) if self.shadow is not None else 0
         st.shadow_col_stride = self.shadow_cs
         st.model_stride = self.model_stride
         st.have_ens = 1 if self.ens is not None else 0
@@ -266,6 +278,10 @@ class Engine:
         st.step_ctr = _ptr(self.step_ctr)
         st.flags = _ptr(self.flags)
         self.st = st
+
+    def _slab_fn(self, name):
+        """C entry point of a pass over the dense slab, for its element type."""
+        return name + "_f16" if self.f16 else name
 
     def _slab_ptr(self):
         return self.preds.data_ptr() if self.compact is None else 0
@@ -286,15 +302,15 @@ class Engine:
                            _ptr(self.pseudo), H, N, C, self.K, self.fx_shift, _ptr(self.conf_fx), _ptr(self.conf_rest), s)
                 self._build_compact_index()
                 return
-            self._call("coda_b200_scan_slab", _ptr(self.preds), self.model_stride, H, N, C, _ptr(self.hard),
+            self._call(self._slab_fn("coda_b200_scan_slab"), _ptr(self.preds), self.model_stride, H, N, C, _ptr(self.hard),
                        _ptr(self.pseudo), _ptr(self.disagree), _ptr(self.ens), _ptr(self.flags), s)
             if C <= 128:
                 order = torch.argsort(self.pseudo).to(torch.int32)      # init-time plumbing: any grouping by label will do
-                self._call("coda_b200_confusion_sorted", _ptr(self.preds), self.model_stride, _ptr(self.pseudo),
+                self._call(self._slab_fn("coda_b200_confusion_sorted"), _ptr(self.preds), self.model_stride, _ptr(self.pseudo),
                            _ptr(order), H, N, C, self.fx_shift, _ptr(self.conf_fx), s)
                 del order
             else:
-                self._call("coda_b200_confusion_accum", _ptr(self.preds), self.model_stride, _ptr(self.pseudo), H, N, C,
+                self._call(self._slab_fn("coda_b200_confusion_accum"), _ptr(self.preds), self.model_stride, _ptr(self.pseudo), H, N, C,
                            self.fx_shift, _ptr(self.conf_fx), s)
 
     def construct_posterior(self):
@@ -370,15 +386,16 @@ class Engine:
         H, N, C, s = self.H, self.N, self.C, self._s()
         if self._pi_tc is None:
             want = os.environ.get("CODA_B200_PI_FULL", "tc") != "simt"
-            self._pi_tc = bool(want and self.lib.coda_b200_pi_full_tc_ok(H, N, C, self.model_stride)
-                               and self.preds.data_ptr() % 16 == 0)
+            # the same views qualify for both element types: an element offset that is a multiple of 4
+            ok = getattr(self.lib, self._slab_fn("coda_b200_pi_full_tc_ok"))
+            self._pi_tc = bool(want and ok(H, N, C, self.model_stride) and self.preds.data_ptr() % (4 * self.esize) == 0)
             if self._pi_tc:
                 self._pi_scratch = self._e((int(self.lib.coda_b200_pi_full_tc_scratch_bytes(H, C)),), torch.uint8)
         if self._pi_tc:
-            self._call("coda_b200_pi_full_tc", _ptr(self.preds), self.model_stride, _ptr(self.D), H, N, C, _ptr(self.U),
+            self._call(self._slab_fn("coda_b200_pi_full_tc"), _ptr(self.preds), self.model_stride, _ptr(self.D), H, N, C, _ptr(self.U),
                        _ptr(self._pi_scratch), _ptr(self.flags), s, n=2)
         else:
-            self._call("coda_b200_pi_full", _ptr(self.preds), self.model_stride, _ptr(self.D), H, N, C, _ptr(self.U), s)
+            self._call(self._slab_fn("coda_b200_pi_full"), _ptr(self.preds), self.model_stride, _ptr(self.D), H, N, C, _ptr(self.U), s)
 
     def _build_rows(self):
         H, N, C, W, T, s = self.H, self.N, self.C, self.W, self.T, self._s()
@@ -455,18 +472,17 @@ class Engine:
                 self.ph_cache = self._e((self.npairs, self.Hp), torch.float32)
 
     def _build_shadow(self):
-        """Class-major shadow copy of as many models as spare HBM allows (least accurate first)."""
+        """Class-major shadow copy of as many models as spare HBM allows (least accurate first), in the slab's element
+        type: an fp16 shadow holds twice the models in the same memory."""
         self.shadow, self.slot_of_model, self.n_shadow, self.shadow_cs = None, None, 0, 0
         if self.mode == "recompute_all" or os.environ.get("CODA_B200_SHADOW", "1") == "0" or self.compact is not None:
             return
         H, N, C = self.H, self.N, self.C
-        cs = (N + 3) // 4 * 4                                   # every (slot, class) column starts 16-byte aligned
         torch.cuda.synchronize(self.dev)
         torch.cuda.empty_cache()
         free, _total = torch.cuda.mem_get_info(self.dev)
         reserve = int(float(os.environ.get("CODA_B200_SHADOW_RESERVE_GB", "8")) * 2 ** 30)
-        per_model = cs * C * 4
-        S = int(min(H, max(0, (free - reserve) // per_model)))
+        S, cs = shadow_slots(free - reserve, H, N, C, self.esize)
         cap = os.environ.get("CODA_B200_SHADOW_MODELS")
         if cap is not None:
             S = min(S, int(cap))
@@ -481,8 +497,8 @@ class Engine:
         order = torch.argsort(dis, descending=True, stable=True)[:S].to(torch.int32)
         slot = torch.full((H,), -1, dtype=torch.int32, device=self.dev)
         slot[order.long()] = torch.arange(S, dtype=torch.int32, device=self.dev)
-        self.shadow = self._e((S, C, cs), torch.float32)
-        self._call("coda_b200_shadow_build", _ptr(self.preds), self.model_stride, H, N, C, _ptr(order), S, cs,
+        self.shadow = self._e((S, C, cs), self.preds.dtype)
+        self._call(self._slab_fn("coda_b200_shadow_build"), _ptr(self.preds), self.model_stride, H, N, C, _ptr(order), S, cs,
                    _ptr(self.shadow), self._s())
         self.slot_of_model, self.n_shadow, self.shadow_cs = slot, S, cs
 
@@ -585,7 +601,7 @@ class Engine:
                        C, self.K, _ptr(self.sel), self.lr, self.fx_shift, _ptr(self.terms), _ptr(self.U),
                        _ptr(self.pisum), _ptr(self.flags), s)
         else:
-            self._call("coda_b200_pi_rank1", _ptr(self.preds), _ptr(self.ens), H, N, C, _ptr(self.sel), self.lr,
+            self._call(self._slab_fn("coda_b200_pi_rank1"), _ptr(self.preds), _ptr(self.ens), H, N, C, _ptr(self.sel), self.lr,
                        self.fx_shift, _ptr(self.terms), _ptr(self.U), _ptr(self.pisum), _ptr(self.flags),
                        4 if fork else 8, self.const_slot, s)
         if fork:

@@ -60,7 +60,9 @@ def _auto_gpus(preds) -> int:
     env = os.environ.get("CODA_B200_GPUS")
     if env:
         return max(1, int(env))
-    if preds.numel() * 4 < (4 << 30):
+    # bytes of the slab: a dense fp16 slab counts 2 per score (the compact form reports its own float count)
+    esize = 2 if getattr(preds, "dtype", None) == torch.float16 else 4
+    if preds.numel() * esize < (4 << 30):
         return 1
     return max(1, torch.cuda.device_count())
 

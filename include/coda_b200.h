@@ -14,6 +14,10 @@
  *     from coda/util.py:17-25 at the same places;
  *   - layouts: preds [H][N][C] fp32 (coda/datasets.py:14), models `model_stride` floats apart (N*C when the
  *     shard is its own tensor; the full-task stride when it is an N-range view of a bigger slab);
+ *   - 16-bit slabs: every entry point that reads preds has an `_f16` twin taking `const uint16_t* preds`, the IEEE
+ *     binary16 bit patterns of the scores in the same layout (strides in elements).  The twins convert on load and
+ *     compute in fp32: their results have the bits of the fp32 entry point on the upcast slab, and they choose
+ *     between kernels exactly as the fp32 entry point does for the same shape and view;
  *     D (dirichlets) [H][C][C] fp32; U (un-normalised pi_hat_xi) [N][C] fp32; hard [N][H] u16;
  *     Hp = H rounded up to 32;
  *   - "rows": one row = one hypothetical (item, class) update.  Rows [0, T), T = C*(1+H), are the template rows
@@ -93,17 +97,24 @@ int coda_b200_peer_enable(int peer_device); /* current device may load/store pee
  * Also util._check_prob (util.py:28-39) on the input: negatives, non-finite values, row sums. */
 int coda_b200_scan_slab(const float* preds, int64_t model_stride, int H, int64_t N, int C, uint16_t* hard,
                         int32_t* pseudo, uint8_t* disagree, float* ens_out, uint32_t* flags, coda_stream_t stream);
+int coda_b200_scan_slab_f16(const uint16_t* preds, int64_t model_stride, int H, int64_t N, int C, uint16_t* hard,
+                            int32_t* pseudo, uint8_t* disagree, float* ens_out, uint32_t* flags, coda_stream_t stream);
 
 /* Soft confusion sums, coda.py:42 einsum('nc,hnj->hcj').  conf_fx [H][C][C] int64 fixed point
  * (value * 2^fx_shift), ACCUMULATED into; exact and order-independent so shards can be summed. */
 int coda_b200_confusion_accum(const float* preds, int64_t model_stride, const int32_t* pseudo, int H, int64_t N,
                               int C, int fx_shift, int64_t* conf_fx, coda_stream_t stream);
+int coda_b200_confusion_accum_f16(const uint16_t* preds, int64_t model_stride, const int32_t* pseudo, int H, int64_t N,
+                                  int C, int fx_shift, int64_t* conf_fx, coda_stream_t stream);
 
 /* Same sums with the items visited in pseudo-label order (`order` = any permutation that groups equal
  * pseudo labels; C <= 128): register accumulation, no shared-memory atomics.  Bit-identical result. */
 int coda_b200_confusion_sorted(const float* preds, int64_t model_stride, const int32_t* pseudo,
                                const int32_t* order, int H, int64_t N, int C, int fx_shift, int64_t* conf_fx,
                                coda_stream_t stream);
+int coda_b200_confusion_sorted_f16(const uint16_t* preds, int64_t model_stride, const int32_t* pseudo,
+                                   const int32_t* order, int H, int64_t N, int C, int fx_shift, int64_t* conf_fx,
+                                   coda_stream_t stream);
 
 /* Row-normalise (coda.py:43) and build the Dirichlet prior (coda.py:46-63, 196). */
 /* conf_rest (optional, compact slab): [H][C] sums every column of row (h, c) carries in addition (see below). */
@@ -116,6 +127,8 @@ int coda_b200_init_dirichlets(const int64_t* conf_fx, const int64_t* conf_rest, 
 /* U[n][c] = sum_h sum_s D[h][c][s] preds[h][n][s]  (coda.py:227-229, `adjusted` never stored). */
 int coda_b200_pi_full(const float* preds, int64_t model_stride, const float* D, int H, int64_t N, int C, float* U,
                       coda_stream_t stream);
+int coda_b200_pi_full_f16(const uint16_t* preds, int64_t model_stride, const float* D, int H, int64_t N, int C, float* U,
+                          coda_stream_t stream);
 
 /* The same contraction on the tensor cores (tcgen05, TMEM accumulators, bulk-TMA slab stream): both operands are cut
  * into two bf16 limbs, 4 MMAs per K = 16 chunk, accumulators drained to fp32 registers every 4 models (pi_tc.cu).
@@ -125,6 +138,10 @@ int coda_b200_pi_full_tc_ok(int H, int64_t N, int C, int64_t model_stride);
 size_t coda_b200_pi_full_tc_scratch_bytes(int H, int C);
 int coda_b200_pi_full_tc(const float* preds, int64_t model_stride, const float* D, int H, int64_t N, int C, float* U,
                          void* scratch, uint32_t* flags, coda_stream_t stream);
+/* fp16: eligible for exactly the shapes of the fp32 pass; preds needs 8-byte alignment (fp32: 16). */
+int coda_b200_pi_full_tc_ok_f16(int H, int64_t N, int C, int64_t model_stride);
+int coda_b200_pi_full_tc_f16(const uint16_t* preds, int64_t model_stride, const float* D, int H, int64_t N, int C,
+                             float* U, void* scratch, uint32_t* flags, coda_stream_t stream);
 
 /* Row-normalise with the 1e-12 clamp (coda.py:230) and accumulate sum_n pi_hat_xi[n][:]
  * (coda.py:232) into pisum_fx [C] (int64 fixed point, ACCUMULATED).  xi_out may be NULL. */
@@ -136,6 +153,11 @@ int coda_b200_pi_reduce(float* U, int64_t N, int C, int fx_shift, float* xi_out,
  * Columns are `col_stride` floats apart (>= N, a multiple of 4 so that every column is 16-byte aligned). */
 int coda_b200_shadow_build(const float* preds, int64_t model_stride, int H, int64_t N, int C,
                            const int32_t* model_of_slot, int S, int64_t col_stride, float* T, coda_stream_t stream);
+/* fp16 shadow of an fp16 slab: col_stride a multiple of 8 (16-byte aligned columns); the step kernels' shadow_off
+ * counts slab ELEMENTS (halves) from preds to T. */
+int coda_b200_shadow_build_f16(const uint16_t* preds, int64_t model_stride, int H, int64_t N, int C,
+                               const int32_t* model_of_slot, int S, int64_t col_stride, uint16_t* T,
+                               coda_stream_t stream);
 
 /* update_pi_hat after the rank-1 change of D (coda.py:319): U[n][t] += lr * sum_h preds[h][n][jvec[h]],
  * then the same normalise + column sums as pi_reduce.  The gather list (`terms`, written by the step kernels
@@ -151,6 +173,11 @@ int coda_b200_shadow_build(const float* preds, int64_t model_stride, int H, int6
 int coda_b200_pi_rank1(const float* preds, const float* ens, int H, int64_t N, int C, const int64_t* sel, double lr,
                        int fx_shift, const int32_t* terms, float* U, int64_t* pisum_fx, uint32_t* flags,
                        int ctas_per_sm, int const_slot, coda_stream_t stream);
+/* fp16 slab (and shadow): the gather list holds element offsets from preds.  The opt-in variants that read the slab as
+ * fp32 words (CODA_B200_R1=tma|v4) return CODA_B200_EINVAL; v1 (default) and v1d are available. */
+int coda_b200_pi_rank1_f16(const uint16_t* preds, const float* ens, int H, int64_t N, int C, const int64_t* sel,
+                           double lr, int fx_shift, const int32_t* terms, float* U, int64_t* pisum_fx, uint32_t* flags,
+                           int ctas_per_sm, int const_slot, coda_stream_t stream);
 
 /* ---- compact slab (BASELINE.json configs[4]: M=1024, N=4e6, C=1000 is 16.4 TB dense; no reference counterpart --
  *      the reference cannot run there, coda.py:227 materialises a second slab) ----------------------------------
